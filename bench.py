@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — 50-step inpainting throughput of the PowerPaint denoising hot path on B200.
 
-    python bench.py --gpus N --steps K --warmup W [--config C2|C3|C4|C5]     (N > 1: launched under torchrun)
+    python bench.py --gpus N --steps K --warmup W [--config C2|C3|C4|C5] [--dump-outputs DIR]   (N > 1: under torchrun)
     python bench.py --impl reference [--gpus N ...]                          CPU arm: the oracle port of the reference
 
 Workloads (BASELINE.json `configs`; every rank runs the per-GPU share, weak scaling):
@@ -352,6 +352,15 @@ def oracle_loop(cfg, ou, side, sched, kw, dtype):
     return loop_v1(ou, sched, c(kw["latents"]), c(kw["prompt_embeds"]), c(ex[:, :1]), c(ex[:, 1:]), GUIDANCE)
 
 
+def write_outputs(directory, arrays):
+    """`--dump-outputs`: one float32 DIR/<name>.npy per array, so that two builds can be compared output for output"""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), t.numpy().astype(np.float32))
+
+
 def run_gpu_arm(args):
     rank, world, local = _dist_env()
     if world != args.gpus and world == 1 and args.gpus > 1:
@@ -403,6 +412,7 @@ def run_gpu_arm(args):
         e1.record()
         barrier()
     assert torch.isfinite(out).all(), "non-finite latents in the timed region"
+    dump = {"latents": out.float().cpu()} if args.dump_outputs and rank == 0 else None
     ms = e0.elapsed_time(e1)
     t = torch.tensor([ms], device=dev)
     if dist is not None:
@@ -459,12 +469,15 @@ def run_gpu_arm(args):
     e2e_once()
     e2e_once()
     barrier()
-    k_e2e = max(3, args.steps)
+    k_e2e = args.steps
     t0 = time.perf_counter()
     for _ in range(k_e2e):
         e2e_once()
     barrier()
     dt = time.perf_counter() - t0
+    if dump is not None:  # rank 0's own shard: the first B of the gathered images
+        dump["images"] = out_host[:B].float()
+        write_outputs(args.dump_outputs, dump)
     tt = torch.tensor([dt], device=dev)
     if dist is not None:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -559,7 +572,13 @@ def main():
     ap.add_argument("--config", default="C2", choices=sorted(CONFIGS))
     ap.add_argument("--no-baselines", action="store_true",
                     help="skip the parity spot check and the CPU / library baselines (profiling runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32, "
+                         "rank 0): latents.npy = the denoising loop's final latents [B,4,h,w], images.npy = the e2e "
+                         "pipeline call's uint8 images [B,H,W,3] as float32")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference_arm(args)
     return run_gpu_arm(args)

@@ -1,6 +1,6 @@
 """Stand-in for `diffusers==0.27.0`, JUST ENOUGH for the reference's own model files
-(`/root/reference/powerpaint/models/{unet_2d_blocks,unet_2d_condition,BrushNet_CA}.py`) and pipeline files
-(`/root/reference/powerpaint/pipelines/pipeline_PowerPaint{,_Brushnet_CA,_ControlNet}.py`: DiffusionPipeline plumbing,
+(`powerpaint/models/{unet_2d_blocks,unet_2d_condition,BrushNet_CA}.py`) and pipeline files
+(`powerpaint/pipelines/pipeline_PowerPaint{,_Brushnet_CA,_ControlNet}.py`: DiffusionPipeline plumbing,
 VaeImageProcessor for tensors, a DDIM scheduler / AutoencoderKL / ControlNetModel that are the oracle's) to import and run
 UNMODIFIED on the CPU, so that golden vectors of the reference's *composition* can be generated here
 (tests/golden/make_unet_golden.py): where BrushNet's 28 adds go, which skip the tuple keeps, how the up path pops,

@@ -1,8 +1,8 @@
 """Generate tests/golden/pipeline_v1_call.npz by running the REFERENCE's own v1 pipeline `__call__`.
 
-    python tests/golden/make_pipeline_golden.py          # needs /root/reference (this container only)
+    PP_REFERENCE_DIR=<checkout of the original PowerPaint project> python tests/golden/make_pipeline_golden.py
 
-`/root/reference/powerpaint/pipelines/pipeline_PowerPaint.py` and the reference UNet are imported UNMODIFIED over
+`powerpaint/pipelines/pipeline_PowerPaint.py` of that checkout and the reference UNet are imported UNMODIFIED over
 tests/golden/diffusers_shim. What the fixture pins is everything `__call__` itself does between the user's arguments and
 the final latents (pipeline_PowerPaint.py:855-1071): `prepare_mask_and_masked_image`, the strength -> timestep window,
 the order of the generator draws (initial noise first, then the VAE posterior sample of the masked image), the mask
@@ -19,7 +19,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-sys.path[:0] = [os.path.join(HERE, "diffusers_shim"), "/root/reference", ROOT]
+sys.path[:0] = [os.path.join(HERE, "diffusers_shim"), os.environ["PP_REFERENCE_DIR"], ROOT]
 
 import types  # noqa: E402
 

@@ -1,9 +1,8 @@
 """Generates tests/golden/token_api.json by running the REFERENCE's own implementation of the
-task-prompt token API (/root/reference/powerpaint/utils/utils.py, imported as is with a one-function
+task-prompt token API (powerpaint/utils/utils.py of the original project, imported as is with a one-function
 `mmengine` stub) on the synthetic CLIP tokenizer / text encoder of synthetic_clip.py.
 
-Run in the build container (the reference tree is not on the GPU box):
-    python tests/golden/make_token_api_golden.py
+    PP_REFERENCE_DIR=<checkout of the original PowerPaint project> python tests/golden/make_token_api_golden.py
 """
 import importlib.util
 import json
@@ -17,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, HERE)
 from synthetic_clip import make_text_encoder, make_tokenizer  # noqa: E402
 
-REF = "/root/reference/powerpaint/utils/utils.py"
+REF = os.path.join(os.environ["PP_REFERENCE_DIR"], "powerpaint", "utils", "utils.py")
 
 PROMPTS = [
     "a photo of a cat P_obj",

@@ -1,8 +1,8 @@
 """Generate tests/golden/unet_composition.npz from the REFERENCE's own model files.
 
-    python tests/golden/make_unet_golden.py          # needs /root/reference (this container only)
+    PP_REFERENCE_DIR=<checkout of the original PowerPaint project> python tests/golden/make_unet_golden.py
 
-`/root/reference/powerpaint/models/{unet_2d_blocks,unet_2d_condition,BrushNet_CA}.py` are imported UNMODIFIED; the absent
+`powerpaint/models/{unet_2d_blocks,unet_2d_condition,BrushNet_CA}.py` of that checkout are imported UNMODIFIED; the absent
 `diffusers` dependency is replaced by tests/golden/diffusers_shim (adapters over oracle/blocks.py for the primitive blocks
 the SD-1.5 configuration instantiates, placeholders for everything else). What this pins is therefore the reference's
 COMPOSITION — the 28 BrushNet add points and their pop(0) order, which states the skip tuple keeps, the up-path pops and
@@ -20,7 +20,7 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-sys.path[:0] = [os.path.join(HERE, "diffusers_shim"), "/root/reference", ROOT]
+sys.path[:0] = [os.path.join(HERE, "diffusers_shim"), os.environ["PP_REFERENCE_DIR"], ROOT]
 
 from powerpaint.models.BrushNet_CA import BrushNetModel as RefBrushNet  # noqa: E402  (the reference, unmodified)
 from powerpaint.models.unet_2d_condition import UNet2DConditionModel as RefUNet  # noqa: E402
@@ -58,6 +58,11 @@ def main():
     for tag, (h, w) in {"8x8": (8, 8), "10x12": (10, 12)}.items():
         x, ctx, _ = inputs(11, 9, h, w)
         out[f"unet9_{tag}"] = u9(x, 321, ctx).sample.numpy()
+    # two more seeds at another timestep, and the parameter names, that the oracle is held to
+    for seed, (h, w) in ((3, (8, 8)), (4, (12, 10))):
+        x, ctx, _ = inputs(seed, 9, h, w)
+        out[f"unet9_seed{seed}_{h}x{w}"] = u9(x, 77, ctx).sample.numpy()
+    out["unet9_state_dict_keys"] = np.array(sorted(u9.state_dict()))
     # ---- v2: BrushNet forward (28 outputs), 4-channel UNet consuming them, from_unet
     u4 = ref_unet(4)
     u4.load_state_dict(synthetic_state_dict(cfg(4), "unet", 1234), strict=True)

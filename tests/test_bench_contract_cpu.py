@@ -52,6 +52,13 @@ def test_reference_arm_times_the_loop_of_the_named_config():
     assert "1024x1024" in bench.cpu_sample_text(bench.CONFIGS["C4"])
 
 
+def test_steps_below_one_are_refused():
+    """--steps is the number of timed steps of every timed region, so zero timed steps is an error, not a line"""
+    r = _run("--steps", "0", timeout=120)
+    assert r.returncode == 2 and "--steps must be at least 1" in r.stderr
+    assert not [ln for ln in r.stdout.splitlines() if ln.startswith("{")]
+
+
 def test_product_arm_refuses_to_run_without_a_gpu():
     import torch
 
