@@ -516,11 +516,14 @@ class NetEngine:
 
     def plan(self, nb: int, h: int, w: int, ctx_len: int = 77, *, with_brushnet_adds: bool = False,
              with_controlnet_res: bool = False, use_step_table: bool = False, n_steps: int = 0,
-             brushnet_outputs: bool = False) -> Plan:
-        key = (nb, h, w, ctx_len, with_brushnet_adds, with_controlnet_res, use_step_table, n_steps, brushnet_outputs)
+             brushnet_outputs: bool = False, guess_mode: bool = False) -> Plan:
+        key = (nb, h, w, ctx_len, with_brushnet_adds, with_controlnet_res, use_step_table, n_steps, brushnet_outputs,
+               guess_mode)
         p = self._plans.pop(key, None)
         if p is None:
-            p = self._build_plan(nb, h, w, ctx_len, with_brushnet_adds, with_controlnet_res, use_step_table, n_steps)
+            shared = dict(cn_alpha=self.guess_alphas()) if guess_mode else None
+            p = self._build_plan(nb, h, w, ctx_len, with_brushnet_adds, with_controlnet_res, use_step_table, n_steps,
+                                 shared=shared)
             if self.kind in ("brushnet", "controlnet") and p.scale_dev is None:
                 # eager forward: conditioning_scale is read from a device scalar at run time
                 p.scale_dev = torch.ones(1, dtype=torch.float32, device=self.device)
@@ -530,6 +533,14 @@ class NetEngine:
                 self._plans.pop(next(iter(self._plans)))
         self._plans[key] = p  # most recently used last
         return p
+
+    def guess_alphas(self):
+        """(down, mid) constant factors of a ControlNet's residuals in guess mode: diffusers' ControlNetModel.forward
+        scales the down residuals by torch.logspace(-1, 0, n_down + 1)[:n_down] and the mid residual by its last
+        entry (1.0), each times conditioning_scale (which stays the device-side factor)"""
+        n_down = len(self._state_shapes(1, 64, 64)[0])
+        s = torch.logspace(-1, 0, n_down + 1, dtype=torch.float32).tolist()
+        return s[:n_down], s[-1]
 
     @staticmethod
     def _levels(h: int, w: int, n: int):
@@ -568,7 +579,9 @@ class NetEngine:
         first channels are this net's input; extra channels meet zero weights), `timesteps`,
         `step_idx`, `plan` (record into an existing Plan so that the nets share one buffer pool), and for the
         UNet `adds` = (down, mid, up) / `cn` = (down, mid) buffers produced by the side net;
-        `scale_dev` = (tensor, step_idx, stride): device-side conditioning scale of the side net."""
+        `scale_dev` = (tensor, step_idx, stride): device-side conditioning scale of the side net; for a ControlNet
+        `cn_out` / `cn_res2` = (down list, mid): buffers its zero-convs write / add after scaling, and
+        `cn_alpha` = (down list, mid): constant per-residual factors (`guess_alphas`)."""
         shared = shared or {}
         cfg = self.cfg
         boc = cfg.block_out_channels
@@ -746,16 +759,22 @@ class NetEngine:
             sdev, sstep, sstride = shared.get("scale_dev") or (plan.scale_dev, None, 0)
             if sdev is None:
                 sdev = plan.scale_dev = torch.ones(1, dtype=torch.float32, device=self.device)
+            # zero-conv outputs: the caller's buffers (`cn_out`), else persistent ones; `cn_res2` (another ControlNet's
+            # residuals) is added after the scale, so chained nets leave the running sum in the last net's outputs;
+            # `cn_alpha`: constant per-residual factors (guess mode) next to the device scale
+            t_down, t_mid = shared.get("cn_out") or ([None] * len(states_down), None)
+            r_down, r_mid = shared.get("cn_res2") or ([None] * len(states_down), None)
+            a_down, a_mid = shared.get("cn_alpha") or ([1.0] * len(states_down), 1.0)
             outs_down = []
             for k, st in enumerate(states_down):
                 c = st.shape[-1]
-                o = persistent(st.numel() // c, c)
+                o = t_down[k] if t_down[k] is not None else persistent(st.numel() // c, c)
                 outs_down.append(self._linear(plan, prog, st, st.numel() // c, f"controlnet_down_blocks.{k}", c,
-                                              bias=self.vec(f"controlnet_down_blocks.{k}.bias"), out=o,
-                                              alpha_dev=sdev, alpha_step=sstep, alpha_stride=sstride))
-            o = persistent(state_mid.numel() // cm, cm)
+                                              bias=self.vec(f"controlnet_down_blocks.{k}.bias"), out=o, res2=r_down[k],
+                                              alpha=a_down[k], alpha_dev=sdev, alpha_step=sstep, alpha_stride=sstride))
+            o = t_mid if t_mid is not None else persistent(state_mid.numel() // cm, cm)
             out_mid = self._linear(plan, prog, state_mid, state_mid.numel() // cm, "controlnet_mid_block",
-                                   cm, bias=self.vec("controlnet_mid_block.bias"), out=o,
+                                   cm, bias=self.vec("controlnet_mid_block.bias"), out=o, res2=r_mid, alpha=a_mid,
                                    alpha_dev=sdev, alpha_step=sstep, alpha_stride=sstride)
             plan.outputs["down"], plan.outputs["mid"] = outs_down, out_mid
             for st in states_down + [state_mid]:

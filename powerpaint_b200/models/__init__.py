@@ -1,8 +1,8 @@
 from .autoencoder_kl import AutoencoderKL
 from .clip_text import CLIPTextModel
 from .unet_2d_condition import (BrushNetModel, BrushNetOutput, ControlNetModel, ControlNetOutput,
-                                UNet2DConditionModel, UNet2DConditionOutput)
+                                MultiControlNetModel, UNet2DConditionModel, UNet2DConditionOutput)
 from .spec import param_shapes, synthetic_state_dict
 
 __all__ = ["AutoencoderKL", "BrushNetModel", "BrushNetOutput", "CLIPTextModel", "ControlNetModel", "ControlNetOutput",
-           "UNet2DConditionModel", "UNet2DConditionOutput", "param_shapes", "synthetic_state_dict"]
+           "MultiControlNetModel", "UNet2DConditionModel", "UNet2DConditionOutput", "param_shapes", "synthetic_state_dict"]

@@ -16,6 +16,7 @@ reference does (unet_2d_condition.py:1223); outputs are fresh tensors in `self.d
 """
 from __future__ import annotations
 
+import os
 from dataclasses import asdict, dataclass
 from types import SimpleNamespace
 from typing import Any, Dict, List, Optional, Tuple, Union
@@ -386,28 +387,119 @@ class ControlNetModel(_HotPathModel):
                 added_cond_kwargs: Optional[Dict[str, torch.Tensor]] = None,
                 cross_attention_kwargs: Optional[Dict[str, Any]] = None, guess_mode: bool = False,
                 return_dict: bool = True):
-        if guess_mode:
-            raise NotImplementedError("guess_mode is outside the PowerPaint hot path")
+        """`guess_mode`: the 12 down residuals are scaled by torch.logspace(-1, 0, 13)[:12] and the mid residual by 1.0,
+        each times `conditioning_scale` (diffusers ControlNetModel.forward); the factors are constants of a plan
+        recorded for guess mode, the scale stays a device scalar."""
         nb, _, h, w = sample.shape
-        if tuple(controlnet_cond.shape[2:]) != (8 * h, 8 * w):
-            raise ValueError("controlnet_cond must be 8x the latent resolution")
         with torch.cuda.device(self.device):
-            eng = self.engine()
-            plan = eng.plan(nb, h, w, encoder_hidden_states.shape[1])
-            # t-independent (SURVEY.md App. C (3)): the 8-conv embedding is re-run only when the staged control
-            # image actually differs (content comparison on the device; an address is not an identity)
-            ci = plan.inputs["cond_in"]
-            new_ci = ops.nchw_to_nhwc(controlnet_cond.float().contiguous(), ci.shape[-1]).view_as(ci)
-            if not plan.outputs.get("cond_valid") or not torch.equal(new_ci, ci):
-                ci.copy_(new_ci)
-                plan.cond_program.run()
-                plan.outputs["cond_valid"] = True
-            plan.scale_dev.fill_(float(conditioning_scale))
-            self._load_inputs(plan, sample, timestep, encoder_hidden_states)
-            plan.program.launch()
-            shapes_d, shape_m, _ = eng._state_shapes(nb, h, w)
-            down = [self._to_nchw(t, nb, sh[1], sh[2], self.dtype) for t, sh in zip(plan.outputs["down"], shapes_d)]
-            mid = self._to_nchw(plan.outputs["mid"], nb, shape_m[1], shape_m[2], self.dtype)
+            outs = self._run(sample, timestep, encoder_hidden_states, controlnet_cond, conditioning_scale, guess_mode)
+            down, mid = self._residuals_nchw(outs, nb, h, w)
         if not return_dict:
             return (down, mid)
         return ControlNetOutput(down_block_res_samples=down, mid_block_res_sample=mid)
+
+    def _run(self, sample, timestep, encoder_hidden_states, controlnet_cond, conditioning_scale, guess_mode):
+        """one forward on the recorded plan: (down, mid) channels-last bf16 residuals owned by the plan"""
+        nb, _, h, w = sample.shape
+        if tuple(controlnet_cond.shape[2:]) != (8 * h, 8 * w):
+            raise ValueError("controlnet_cond must be 8x the latent resolution")
+        eng = self.engine()
+        plan = eng.plan(nb, h, w, encoder_hidden_states.shape[1], guess_mode=bool(guess_mode))
+        # t-independent (SURVEY.md App. C (3)): the 8-conv embedding is re-run only when the staged control
+        # image actually differs (content comparison on the device; an address is not an identity)
+        ci = plan.inputs["cond_in"]
+        new_ci = ops.nchw_to_nhwc(controlnet_cond.float().contiguous(), ci.shape[-1]).view_as(ci)
+        if not plan.outputs.get("cond_valid") or not torch.equal(new_ci, ci):
+            ci.copy_(new_ci)
+            plan.cond_program.run()
+            plan.outputs["cond_valid"] = True
+        plan.scale_dev.fill_(float(conditioning_scale))
+        self._load_inputs(plan, sample, timestep, encoder_hidden_states)
+        plan.program.launch()
+        return plan.outputs["down"], plan.outputs["mid"]
+
+    def _residuals_nchw(self, outs, nb, h, w):
+        shapes_d, shape_m, _ = self.engine()._state_shapes(nb, h, w)
+        down = [self._to_nchw(t, nb, sh[1], sh[2], self.dtype) for t, sh in zip(outs[0], shapes_d)]
+        return down, self._to_nchw(outs[1], nb, shape_m[1], shape_m[2], self.dtype)
+
+
+class MultiControlNetModel(nn.Module):
+    """diffusers' `MultiControlNetModel`: several ControlNets whose residuals are summed (net 0 first). The reference
+    pipeline wraps a list / tuple of ControlNets in it (ref:pipeline_PowerPaint_ControlNet.py:306)."""
+
+    def __init__(self, controlnets):
+        super().__init__()
+        self.nets = nn.ModuleList(controlnets)
+
+    @property
+    def config(self):
+        return self.nets[0].config
+
+    @property
+    def generation(self) -> tuple:
+        """changes whenever the parameters of any net change"""
+        return tuple(n.generation for n in self.nets)
+
+    @property
+    def dtype(self) -> torch.dtype:
+        return self.nets[0].dtype
+
+    @property
+    def device(self) -> torch.device:
+        return self.nets[0].device
+
+    def to(self, *args, **kwargs):
+        for n in self.nets:
+            n.to(*args, **kwargs)
+        return self
+
+    @torch.no_grad()
+    def forward(self, sample: torch.FloatTensor, timestep: Union[torch.Tensor, float, int],
+                encoder_hidden_states: torch.Tensor, controlnet_cond: List[torch.Tensor],
+                conditioning_scale: List[float], class_labels: Optional[torch.Tensor] = None,
+                timestep_cond: Optional[torch.Tensor] = None, attention_mask: Optional[torch.Tensor] = None,
+                added_cond_kwargs: Optional[Dict[str, torch.Tensor]] = None,
+                cross_attention_kwargs: Optional[Dict[str, Any]] = None, guess_mode: bool = False,
+                return_dict: bool = True):
+        """zips images, scales and nets like diffusers (a shorter list runs fewer nets); returns (down, mid)"""
+        for name, v in (("class_labels", class_labels), ("timestep_cond", timestep_cond),
+                        ("attention_mask", attention_mask), ("added_cond_kwargs", added_cond_kwargs)):
+            if v is not None:
+                raise NotImplementedError(f"`{name}` is outside the PowerPaint SD-1.5 hot path")
+        if cross_attention_kwargs:
+            raise NotImplementedError("cross_attention_kwargs are outside the hot path")
+        nb, _, h, w = sample.shape
+        total = None
+        with torch.cuda.device(self.device):
+            for image, scale, net in zip(controlnet_cond, conditioning_scale, self.nets):
+                d, m = net._run(sample, timestep, encoder_hidden_states, image, scale, guess_mode)
+                if total is None:  # the plan owns its outputs: the sum lives in buffers of its own
+                    total = ([t.clone() for t in d], m.clone())
+                else:  # bf16 + bf16 -> bf16, the rounding of the fused loop's chained zero-convs
+                    for acc, t in zip(total[0], d):
+                        ops.add(acc, t, acc)
+                    ops.add(total[1], m, total[1])
+            if total is None:
+                raise ValueError("no ControlNet ran: controlnet_cond / conditioning_scale are empty")
+            return self.nets[0]._residuals_nchw(total, nb, h, w)
+
+    def save_pretrained(self, save_directory, **kwargs):
+        """net k goes to `save_directory` + ("" if k == 0 else f"_{k}") (diffusers layout)"""
+        save_directory = os.fspath(save_directory)
+        for k, net in enumerate(self.nets):
+            net.save_pretrained(save_directory + ("" if k == 0 else f"_{k}"), **kwargs)
+
+    @classmethod
+    def from_pretrained(cls, pretrained_model_path, **kwargs):
+        """loads `path`, `path_1`, `path_2`, ... until one is missing"""
+        pretrained_model_path = os.fspath(pretrained_model_path)
+        nets, k, path = [], 0, pretrained_model_path
+        while os.path.isdir(path):
+            nets.append(ControlNetModel.from_pretrained(path, **kwargs))
+            k += 1
+            path = pretrained_model_path + f"_{k}"
+        if not nets:
+            raise ValueError(f"No ControlNets found under {os.path.dirname(pretrained_model_path)}. Expected at least "
+                             f"{pretrained_model_path + '_0'}.")
+        return cls(nets)

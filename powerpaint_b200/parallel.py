@@ -120,10 +120,16 @@ def gather_batch(local: torch.Tensor, total: int, dst: int = 0, group=None) -> O
 def _split_batched(batched: dict, total: int):
     """full-batch keywords -> (names, halves, tensors) to scatter; a [2 x total] keyword ([negative; positive], the
     BrushNet pipeline's `prompt_embedsU`) travels as two [total] tensors (halves 1 and 2) so that each half is sharded
-    like the images; halves == 0 marks an ordinary [total] keyword"""
+    like the images; a list of [total] tensors (one control image per ControlNet) travels element by element
+    (halves == 3); halves == 0 marks an ordinary [total] keyword"""
     names, halves, tensors = [], [], []
     for k, v in batched.items():
-        if v.shape[0] == total:
+        if isinstance(v, (list, tuple)):
+            for t in v:
+                if t.shape[0] != total:
+                    raise ValueError(f"`{k}`: batch {t.shape[0]} of a list entry is not the request's {total}")
+                names.append(k), halves.append(3), tensors.append(t)
+        elif v.shape[0] == total:
             names.append(k), halves.append(0), tensors.append(v)
         elif v.shape[0] == 2 * total:
             names += [k, k]
@@ -138,7 +144,10 @@ def _merge_shards(names, halves, shards) -> dict:
     """inverse of `_split_batched` on one rank's shards: the two halves of a stacked keyword are concatenated again"""
     kw = {}
     for k, half, t in zip(names, halves, shards):
-        kw[k] = torch.cat([kw[k], t]) if half == 2 else t
+        if half == 3:
+            kw.setdefault(k, []).append(t)
+        else:
+            kw[k] = torch.cat([kw[k], t]) if half == 2 else t
     return kw
 
 
@@ -151,14 +160,16 @@ def sharded_call(pipe, batched: Optional[dict], device, seeds: Optional[Sequence
     `src` gets the images of the whole batch in request order (others None). `seeds[i]` seeds the generator of GLOBAL
     image i, so the result does not depend on the number of ranks. A rank whose shard is empty skips the call.
     Keywords whose batch is 2 x total (the BrushNet pipeline's `prompt_embedsU` = [negative; positive]) are split per
-    half."""
+    half; a list of full-batch tensors (`control_image` of several ControlNets) is scattered entry by entry and arrives
+    as a list."""
     import torch.distributed as dist
 
     world, rank = dist.get_world_size(group), dist.get_rank(group)
     if rank == src:
         if not batched:
             raise ValueError("rank `src` must pass the batched keywords")
-        total = int((batched["image"] if "image" in batched else next(iter(batched.values()))).shape[0])
+        first = batched["image"] if "image" in batched else next(iter(batched.values()))
+        total = int((first[0] if isinstance(first, (list, tuple)) else first).shape[0])
         names, halves, tensors = _split_batched(batched, total)
         head = [(names, halves, total, None if seeds is None else [int(s) for s in seeds])]
         if seeds is not None and len(seeds) != total:

@@ -156,12 +156,16 @@ def check_prompt_arguments(prompt, negative_prompt, prompt_embeds, negative_prom
                              f"`negative_prompt_embeds` {negative_prompt_embeds.shape}.")
 
 
-def check_control_guidance(control_guidance_start, control_guidance_end):
-    """ref:pipeline_PowerPaint_Brushnet_CA.py:836-855, ref:pipeline_PowerPaint_ControlNet.py:768-786"""
+def check_control_guidance(control_guidance_start, control_guidance_end, n_nets: Optional[int] = None):
+    """ref:pipeline_PowerPaint_Brushnet_CA.py:836-855, ref:pipeline_PowerPaint_ControlNet.py:768-786; `n_nets`: the
+    number of ControlNets of a MultiControlNetModel (one window per net)"""
     if len(control_guidance_start) != len(control_guidance_end):
         raise ValueError(f"`control_guidance_start` has {len(control_guidance_start)} elements, but "
                          f"`control_guidance_end` has {len(control_guidance_end)} elements. Make sure to provide the "
                          "same number of elements to each list.")
+    if n_nets is not None and len(control_guidance_start) != n_nets:
+        raise ValueError(f"`control_guidance_start`: {control_guidance_start} has {len(control_guidance_start)} elements "
+                         f"but there are {n_nets} controlnets available. Make sure to provide {n_nets}.")
     for start, end in zip(control_guidance_start, control_guidance_end):
         if start >= end:
             raise ValueError(f"control guidance start: {start} cannot be larger or equal to control guidance end: "

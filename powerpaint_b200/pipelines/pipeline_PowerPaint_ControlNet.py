@@ -5,8 +5,12 @@ The loop (:1663-1735: ControlNet on the 4-channel latents + control image, 9-cha
 (`FusedDenoiser(mode="controlnet")`); the t-independent `controlnet_cond_embedding(control_image)`
 is evaluated once per call instead of once per step (SURVEY.md App. C (3)).
 
-Out of scope like upstream's dead code: `predict_woControl` (:996-1345, a buggy copy of the v1
-`__call__`), MultiControlNet, guess_mode.
+A list or tuple of ControlNets is wrapped in a `MultiControlNetModel` (:306): one control image, conditioning scale and
+control_guidance window per net, residuals summed in net order inside the recorded step. `guess_mode` (or a ControlNet
+whose config sets `global_pool_conditions`) runs the ControlNets on the conditional half of the CFG batch with
+diffusers' logspace residual scales (:1669-1700).
+
+Out of scope like upstream's dead code: `predict_woControl` (:996-1345, a buggy copy of the v1 `__call__`).
 """
 from __future__ import annotations
 
@@ -15,7 +19,7 @@ from typing import Callable, List, Optional, Union
 import torch
 
 from ..denoise import FusedDenoiser
-from ..models.unet_2d_condition import ControlNetModel, UNet2DConditionModel
+from ..models.unet_2d_condition import ControlNetModel, MultiControlNetModel, UNet2DConditionModel
 from .common import (StableDiffusionPipelineOutput, check_control_guidance, check_image, check_prompt_arguments,
                      decode_latents, prepare_mask_and_masked_image, preprocess_image, randn_tensor,
                      uint8_device_inputs)
@@ -28,13 +32,14 @@ class StableDiffusionControlNetInpaintPipeline(StableDiffusionInpaintPipeline):
         super().__init__(vae, text_encoder, tokenizer, unet, scheduler, safety_checker, feature_extractor,
                          requires_safety_checker)
         if isinstance(controlnet, (list, tuple)):
-            raise NotImplementedError("MultiControlNet is outside the hot path")
+            controlnet = MultiControlNetModel(controlnet)
         self.controlnet = controlnet
         self._denoiser_side = None
 
     def denoiser(self) -> FusedDenoiser:
-        if not isinstance(self.unet, UNet2DConditionModel) or not isinstance(self.controlnet, ControlNetModel):
-            assert False, "unet / controlnet must be powerpaint_b200 UNet2DConditionModel / ControlNetModel"
+        nets = self.controlnet.nets if isinstance(self.controlnet, MultiControlNetModel) else [self.controlnet]
+        if not isinstance(self.unet, UNet2DConditionModel) or not all(isinstance(n, ControlNetModel) for n in nets):
+            assert False, "unet / controlnet must be powerpaint_b200 UNet2DConditionModel / ControlNetModel(s)"
         if self._denoiser is None or self._denoiser_unet is not self.unet or self._denoiser_side is not self.controlnet:
             self._denoiser = FusedDenoiser(self.unet, self.controlnet, mode="controlnet")
             self._denoiser_unet, self._denoiser_side = self.unet, self.controlnet
@@ -51,12 +56,29 @@ class StableDiffusionControlNetInpaintPipeline(StableDiffusionInpaintPipeline):
             raise ValueError(f"`callback_steps` has to be a positive integer but is {callback_steps} of type"
                              f" {type(callback_steps)}.")
         check_prompt_arguments(prompt, negative_prompt, prompt_embeds, negative_prompt_embeds)
-        if not isinstance(self.controlnet, ControlNetModel):
+        if isinstance(self.controlnet, ControlNetModel):
+            check_image(image, prompt, prompt_embeds)
+            if not isinstance(controlnet_conditioning_scale, float):
+                raise TypeError("For single controlnet: `controlnet_conditioning_scale` must be type `float`.")
+            check_control_guidance(control_guidance_start, control_guidance_end)
+            return
+        if not isinstance(self.controlnet, MultiControlNetModel):
             assert False
-        check_image(image, prompt, prompt_embeds)
-        if not isinstance(controlnet_conditioning_scale, float):
-            raise TypeError("For single controlnet: `controlnet_conditioning_scale` must be type `float`.")
-        check_control_guidance(control_guidance_start, control_guidance_end)
+        n = len(self.controlnet.nets)
+        if not isinstance(image, list):
+            raise TypeError("For multiple controlnets: `image` must be type `list`")
+        elif any(isinstance(i, list) for i in image):
+            raise ValueError("A single batch of multiple conditionings are supported at the moment.")
+        elif len(image) != n:
+            raise ValueError(f"For multiple controlnets: `image` must have the same length as the number of "
+                             f"controlnets, but got {len(image)} images and {n} ControlNets.")
+        for image_ in image:
+            check_image(image_, prompt, prompt_embeds)
+        # (the reference's length check of a list scale is unreachable, :757-764: a shorter list runs fewer nets)
+        if isinstance(controlnet_conditioning_scale, list):
+            if any(isinstance(i, list) for i in controlnet_conditioning_scale):
+                raise ValueError("A single batch of multiple conditionings are supported at the moment.")
+        check_control_guidance(control_guidance_start, control_guidance_end, n)
 
     def check_image(self, image, prompt, prompt_embeds):
         """ref:pipeline_PowerPaint_ControlNet.py:788-827"""
@@ -100,19 +122,19 @@ class StableDiffusionControlNetInpaintPipeline(StableDiffusionInpaintPipeline):
                  control_guidance_end: Union[float, List[float]] = 1.0):
         height, width = self._default_height_width(height, width, image)
         prompt, negative_prompt = promptA, negative_promptA
+        multi = isinstance(self.controlnet, MultiControlNetModel)
         # align format for control guidance (:1491-1502), then the reference's checks (:1505-1517)
         if not isinstance(control_guidance_start, list) and isinstance(control_guidance_end, list):
             control_guidance_start = len(control_guidance_end) * [control_guidance_start]
         elif not isinstance(control_guidance_end, list) and isinstance(control_guidance_start, list):
             control_guidance_end = len(control_guidance_start) * [control_guidance_end]
         elif not isinstance(control_guidance_start, list) and not isinstance(control_guidance_end, list):
-            control_guidance_start, control_guidance_end = [control_guidance_start], [control_guidance_end]
+            mult = len(self.controlnet.nets) if multi else 1
+            control_guidance_start, control_guidance_end = mult * [control_guidance_start], mult * [control_guidance_end]
         self.check_inputs_controlnet(prompt, control_image, height, width, callback_steps, negative_prompt,
                                      prompt_embeds, negative_prompt_embeds, controlnet_conditioning_scale,
                                      control_guidance_start, control_guidance_end)
         # valid for the reference, outside the hot path here
-        if guess_mode:
-            raise NotImplementedError("guess_mode is outside the hot path")
         if cross_attention_kwargs:
             raise NotImplementedError("cross_attention_kwargs (LoRA scale) is outside the hot path")
         if prompt is not None and isinstance(prompt, str):
@@ -123,12 +145,19 @@ class StableDiffusionControlNetInpaintPipeline(StableDiffusionInpaintPipeline):
             batch_size = prompt_embeds.shape[0]
         device = self._execution_device
         do_cfg = guidance_scale > 1.0
+        if multi and isinstance(controlnet_conditioning_scale, float):
+            controlnet_conditioning_scale = [controlnet_conditioning_scale] * len(self.controlnet.nets)
+        guess_mode = guess_mode or self.controlnet.config.global_pool_conditions  # (:1536-1541)
         prompt_embeds = self._encode_prompt(promptA, promptB, tradoff, device, num_images_per_prompt, do_cfg,
                                             negative_promptA, negative_promptB, tradoff_nag,
                                             prompt_embeds=prompt_embeds, negative_prompt_embeds=negative_prompt_embeds)
         total = batch_size * num_images_per_prompt
-        control = self.prepare_control_image(control_image, width, height, total, num_images_per_prompt, device,
-                                             torch.float32, do_cfg)
+        if multi:
+            control = [self.prepare_control_image(c, width, height, total, num_images_per_prompt, device, torch.float32,
+                                                  do_cfg, guess_mode) for c in control_image]
+        else:
+            control = self.prepare_control_image(control_image, width, height, total, num_images_per_prompt, device,
+                                                 torch.float32, do_cfg, guess_mode)
         if uint8_device_inputs(self.vae, image, mask):  # see StableDiffusionInpaintPipeline.__call__
             if image.shape[-2:] != mask.shape[-2:] or image.shape[0] != mask.shape[0] or mask.shape[1] != 1:
                 raise ValueError("uint8 image [B,3,H,W] and mask [B,1,H,W] must agree in batch and size")
@@ -154,10 +183,10 @@ class StableDiffusionControlNetInpaintPipeline(StableDiffusionInpaintPipeline):
         mask, masked_image_latents = self.prepare_mask_latents(mask, masked_image, total, height, width, torch.float32,
                                                                device, generator, do_cfg)
         extra_step_kwargs = self.prepare_extra_step_kwargs(generator, eta)
-        keep = [1.0 - float(i / len(timesteps) < control_guidance_start[0]
-                            or (i + 1) / len(timesteps) > control_guidance_end[0]) for i in range(len(timesteps))]
+        keep = [[1.0 - float(i / len(timesteps) < s or (i + 1) / len(timesteps) > e) for i in range(len(timesteps))]
+                for s, e in zip(control_guidance_start, control_guidance_end)]
         # `controlnet_keep` (ref:pipeline_PowerPaint_ControlNet.py:1652-1658): the per-step scale
-        # conditioning_scale * keep[i] sits in the device coefficient table the recorded program indexes
+        # conditioning_scale * keep[i] of each net sits in the device side-scale table the recorded program indexes
         coef = self.scheduler.step_coefficients(timesteps, eta=extra_step_kwargs.get("eta", 0.0))
         ucoef = None
         if getattr(self.scheduler, "kind", "ddim") == "unipc":
@@ -174,11 +203,18 @@ class StableDiffusionControlNetInpaintPipeline(StableDiffusionInpaintPipeline):
                 if i % callback_steps == 0:
                     callback(i, t, lat)
                 return None
+        if multi:
+            # MultiControlNetModel.forward zips images, scales and nets: a shorter scale list runs fewer nets
+            n = min(len(control), len(controlnet_conditioning_scale))
+            side = dict(control_image=control[:n], side_scale=[float(v) for v in controlnet_conditioning_scale[:n]],
+                        side_keep=keep[:n])
+        else:
+            side = dict(control_image=control, side_scale=float(controlnet_conditioning_scale), side_keep=keep[0])
+        if guess_mode:  # only passed when used: single-net callers see the keywords they always did
+            side["guess_mode"] = True
         latents = self.denoiser().run(latents=latents, prompt_embeds=prompt_embeds, side_prompt_embeds=prompt_embeds,
-                                      control_image=control, timesteps=timesteps, coef=coef,
-                                      guidance_scale=guidance_scale,
-                                      extra=torch.cat([mask, masked_image_latents], dim=1),
-                                      side_scale=float(controlnet_conditioning_scale), side_keep=keep,
+                                      timesteps=timesteps, coef=coef, guidance_scale=guidance_scale,
+                                      extra=torch.cat([mask, masked_image_latents], dim=1), **side,
                                       noise_fn=noise_fn, ucoef=ucoef, callback=cb)
         image_o = latents if output_type == "latent" else decode_latents(self.vae, latents, output_type)
         if not return_dict:
